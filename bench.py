@@ -4,6 +4,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (N>1: launched under torch.distributed.run)
   python bench.py --impl reference --gpus N --steps K --warmup W
+  python bench.py --gpus N --steps K --warmup W --dump-outputs DIR    (also writes DIR/G.npy, DIR/b.npy)
 
 A "step" = one pass of the hot path over one batch of synthetic input: begin(active set) ->
 accumulate(shard) -> finish (one ncclAllReduce of [G;b;status] across ranks).
@@ -38,6 +39,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 METRIC = "train_points_per_sec"
 UNIT = "points/s"
@@ -257,7 +259,7 @@ def run_ours(args):
         sampler.start()
     prim = primary_workload(world)
 
-    def measure(name: str, with_e2e: bool, steps: int, warmup: int, precision=None):
+    def measure(name: str, with_e2e: bool, steps: int, warmup: int, precision=None, keep_outputs=False):
         eng.set_precision(sg._native.SGP_PREC_AUTO if precision is None else precision)
         w = WORKLOADS[name]
         n, d, m = w["n_per_gpu"], w["d"], w["m"]
@@ -296,6 +298,10 @@ def run_ours(args):
         launches = eng.launch_count() - launches0
         res = {"name": name, "n": n, "d": d, "m": m, "dev_ms": dev_ms, "kern_ms": kern_ms, "kern_n": kern_n,
                "launches": launches, "t_wall": (t_wall0, t_wall1), "path": path, "e2e_ms": None}
+        if keep_outputs:
+            # the last timed step's all-reduced statistics, as a caller receives them: finishing a finished window
+            # only copies the device-resident [G;b] out (no second all-reduce)
+            res["outputs"] = dict(zip(("G", "b"), eng.finish()))
 
         # tail (m x m, fp64; rank 0 does it in a fit): statistics of the last step are still on the device
         eng.magic(copy_out=False)                       # first call pays cuSOLVER's lazy initialisation / workspace
@@ -377,7 +383,11 @@ def run_ours(args):
         return e
 
     other = "configs1" if prim == "configs3" else "configs3"
-    rp = measure(prim, True, args.steps, args.warmup)
+    rp = measure(prim, True, args.steps, args.warmup, keep_outputs=bool(args.dump_outputs) and rank == 0)
+    if "outputs" in rp:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for k, v in rp.pop("outputs").items():
+            np.save(os.path.join(args.dump_outputs, k + ".npy"), v)
     ro = measure(other, False, max(2, min(args.steps, 3)), 3)
     clocks = sampler.stop(*rp["t_wall"]) if rank == 0 else None
     rd = None
@@ -505,7 +515,15 @@ def main():
     ap.add_argument("--no-sweep", dest="sweep", action="store_false", help="skip the K_nm sweep number (N=1 only)")
     ap.add_argument("--no-direct", dest="direct", action="store_false",
                     help="skip the direct-distance int8 series entry (N=1 only)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the statistics of the last timed step of the primary workload as DIR/G.npy (m x m) and "
+                         "DIR/b.npy (m), float64: at most 32 MB (m = 2000); the inputs are seeded, so two builds can be "
+                         "compared output for output")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:
