@@ -158,7 +158,7 @@ typedef struct {
 
 /* nll = sum_e [ 1/2 y_e^T K_e^-1 y_e + 1/2 log|det K_e| ]  and its gradient (n_hypers entries), summed over the
  * uploaded experts and over ranks (ncclAllReduce of 1 + n_hypers doubles + a status word if a communicator exists).
- * Experts of any size (GaussianProcessParams.scala:36 sets no bound).  Fast path: on-chip Cholesky per expert (<= ~165
+ * Experts of any size (GaussianProcessParams.scala:36 sets no bound).  Fast path: on-chip Cholesky per expert (<= 168
  * points, SPD).  When an expert is larger, or a Cholesky pivot is not positive, the evaluation runs the reference's own
  * arithmetic instead -- LU with partial pivoting, log|det| with the sign dropped (logDetAndInv.scala:36-63, GPR:59) --
  * and only an exactly singular matrix fails, with SGP_E_SINGULAR (Breeze's MatrixSingularException). */

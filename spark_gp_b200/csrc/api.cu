@@ -753,7 +753,7 @@ int sgp_experts_upload(sgp_ctx* h, const double* X, const double* y, const int64
     if (ne <= 0) return fail(c, SGP_E_BADARG, "empty expert");
     if (ne > nmax) nmax = static_cast<int>(ne);
   }
-  // (no upper bound on the expert size -- GaussianProcessParams.scala:36: experts above the on-chip kernel's ~165 points
+  // (no upper bound on the expert size -- GaussianProcessParams.scala:36: experts above the on-chip kernel's 168 points
   //  take the global-memory LU path of sgp_bcm_nll)
   SGP_CUDA(c, cudaStreamSynchronize(c->stream));
   cudaFree(c->dEx); cudaFree(c->dEy); cudaFree(c->dEoff); cudaFree(c->dEf);
@@ -948,7 +948,7 @@ int sgp_bcm_nll(sgp_ctx* h, const sgp_kernel_desc* k, const sgp_hyper* hypers, i
   ObjectiveArgs o;
   int rc = objective_setup(c, k, hypers, nh, o);
   if (rc != SGP_OK) return rc;
-  // fast path: on-chip Cholesky per expert (SPD kernel matrices of <= ~165 points -- every default configuration).
+  // fast path: on-chip Cholesky per expert (SPD kernel matrices of <= 168 points -- every default configuration).
   // general path: experts of any size, or a kernel matrix on which Cholesky broke down (not positive definite): the
   // reference's own arithmetic, LU with partial pivoting and log|det| with the sign dropped (logDetAndInv.scala:36-63,
   // GPR:59), on kernel matrices staged in global memory.  The choice is rank-local; the one all-reduce per evaluation
@@ -989,7 +989,7 @@ int sgp_laplace_nll(sgp_ctx* h, const sgp_kernel_desc* k, const sgp_hyper* hyper
   int rc = objective_setup(c, k, hypers, nh, o);
   if (rc != SGP_OK) return rc;
   if (laplace_smem_bytes(c->ex_nmax) > 227 * 1024)
-    return fail(c, SGP_E_BADARG, "datasetSizeForExpert too large for the on-chip Laplace kernel (max ~115 points per expert)");
+    return fail(c, SGP_E_BADARG, "datasetSizeForExpert too large for the on-chip Laplace kernel (max 117 points per expert)");
   SGP_CUDA(c, launch_laplace(c->dEx, c->dEy, c->dEf, c->dEoff, c->n_experts, c->ex_d, c->ex_nmax, o.kf, o.dBeta, nh,
                              o.dKind, o.dTerm, o.dDim, o.dCoef, o.dValue, o.any_ard, tol, c->dNllPer, o.dTotal, o.dFlags, c->stream));
   c->launches += 2;
